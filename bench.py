@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Llama-3-8B-shaped 4-bit (gs=64, axis=1) decode tokens/s on B200 through hqq_b200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" is one decoded token (bs=1, seq=1) through all 32 blocks + lm_head of a random-init Llama-3-8B-shaped
@@ -14,6 +14,10 @@ all-reduce with HQQ_B200_TP_MODE=nccl), i.e. strong scaling.
 
 `--impl reference` times the reference algorithm's CPU implementation (the oracle port of HQQBackend.PYTORCH:
 dequantise -> matmul per linear) on this box's host cores on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes what the last timed step of the device-resident loop handed its caller: DIR/next_token.npy (the
+greedy token of every sequence, float64) and DIR/logits.npy (float32 [batch, vocab]).  The weights come from fixed seeds and
+decoding starts from a fixed token, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -468,6 +472,28 @@ def tokens_agree(model, torch, n_tokens=16):
     return bool(flag.item()), detail
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, next_tok, logits, rank, world):
+    """--dump-outputs: the greedy tokens [batch] as float64 and the logits [batch, vocab] as float32 in `out_dir`.  With tp > 1 the
+    ranks' vocabulary shards are gathered first.  Above DUMP_BYTES only the first sequences are kept (every sequence of the bench
+    starts from the same token, so they are a fixed sample of the batch)."""
+    import numpy as np
+    if world > 1:
+        import torch
+        import torch.distributed as dist
+        parts = [torch.empty_like(logits) for _ in range(world)]
+        dist.all_gather(parts, logits.contiguous())
+        logits = torch.cat(parts, dim=-1)
+    if rank != 0:
+        return
+    rows = max(1, DUMP_BYTES // (4 * logits.shape[-1]))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "next_token.npy"), next_tok[:rows].cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "logits.npy"), logits[:rows].float().cpu().numpy())
+
+
 def run_gpu(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -535,6 +561,8 @@ def run_gpu(args, rank, world, local_rank):
     e1.record(stream)
     barrier()
     dev_ms = e0.elapsed_time(e1)
+    # the next loop overwrites the step's buffers: keep what the last timed step produced
+    last = (model.next_tok.clone(), model._bufs["logits"].clone()) if args.dump_outputs else None
 
     # ---- end-to-end loop through the public API with host buffers ------------------------------
     h_in = torch.ones(B, dtype=torch.long).pin_memory()
@@ -561,6 +589,8 @@ def run_gpu(args, rank, world, local_rank):
         t = torch.tensor([dev_ms, e2e_ms], device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         dev_ms, e2e_ms = t.tolist()
+    if last is not None:
+        dump_outputs(args.dump_outputs, *last, rank, world)
 
     peaks = load_peaks()
     roof = kernel_roofline(model, torch, peaks) if (rank == 0 and B == 1) else None
@@ -660,7 +690,12 @@ def main():
     ap.add_argument("--batch", type=int, default=1, help="sequences decoded in lock-step (BASELINE configs[4]: 32); > 1 runs the small-M / tcgen05 "
                     "kernels between the batched glue kernels, NCCL all-reduce for the tensor-parallel partials")
     ap.add_argument("--model", default="8b", choices=["8b", "70b"], help="70b = BASELINE configs[4] (use with --gpus 8)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the last timed step's tokens and logits to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm (--impl hqq_b200)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

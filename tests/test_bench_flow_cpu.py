@@ -7,6 +7,7 @@ import json
 import os
 import types
 
+import numpy as np
 import pytest
 import torch
 
@@ -15,8 +16,15 @@ from hqq_b200 import harness
 
 
 class FakeGraph:
+    """A replay counts the steps: step n produces token n and logits filled with n."""
+    def __init__(self, model):
+        self.model = model
+
     def replay(self):
-        pass
+        m = self.model
+        m.replays += 1
+        m.next_tok.fill_(m.replays)
+        m._bufs["logits"].fill_(m.replays)
 
 
 class FakeModel:
@@ -25,8 +33,10 @@ class FakeModel:
     def __init__(self, shape, **kw):
         self.kw, self.shape = kw, shape
         self.device, self.dtype, self.nbits, self.tp_mode = torch.device("cpu"), torch.float16, 4, "p2p"
-        self.tok, self.pos, self.next_tok = torch.zeros(1, dtype=torch.long), torch.zeros(1, dtype=torch.long), torch.zeros(1, dtype=torch.long)
-        self.graph, self.blocks = FakeGraph(), []
+        B = kw.get("batch", 1)
+        self.tok, self.pos, self.next_tok = torch.zeros(B, dtype=torch.long), torch.zeros(1, dtype=torch.long), torch.zeros(B, dtype=torch.long)
+        self._bufs, self.replays = {"logits": torch.zeros(B, 8, dtype=torch.float16)}, 0
+        self.graph, self.blocks = FakeGraph(self), []
         FakeModel.built.append(self)
 
     def capture(self, warmup=3):
@@ -36,7 +46,7 @@ class FakeModel:
         pass
 
     def decode(self, feed_back=True):
-        pass
+        self.graph.replay()
 
     def bytes_per_token(self):
         return 4.98e9
@@ -86,7 +96,7 @@ def fake_gpu(monkeypatch):
 
 def _args(**kw):
     d = dict(gpus=1, steps=20, warmup=3, impl="hqq_b200", cache_len=0, layers=0, no_cpu_baseline=False, no_extras=False, quick_extras=False,
-             no_token_check=False, extras_deadline=60.0, batch=1, model="8b")
+             no_token_check=False, extras_deadline=60.0, batch=1, model="8b", dump_outputs=None)
     d.update(kw)
     return argparse.Namespace(**d)
 
@@ -121,6 +131,30 @@ def test_run_gpu_keeps_the_line_when_an_extra_object_fails(fake_gpu, capsys, mon
     bench.run_gpu(_args(no_cpu_baseline=True), 0, 1, 0)
     d = json.loads([ln for ln in capsys.readouterr().out.splitlines() if ln.startswith("{")][-1])
     assert "sweep failed" in d["roofline"]["gemm"]["error"] and d["value"] > 0 and d["roofline"]["quantizer"]["ms_per_block"] == 1.5
+
+
+def test_dump_outputs_holds_the_last_timed_step(fake_gpu, capsys, tmp_path, monkeypatch):
+    """3 warm-up + 20 timed steps in the device loop: the dump is step 23, not what the end-to-end loop replays after it."""
+    out = tmp_path / "dump"
+    bench.run_gpu(_args(no_extras=True, dump_outputs=str(out)), 0, 1, 0)
+    tok, logits = np.load(out / "next_token.npy"), np.load(out / "logits.npy")
+    assert tok.dtype == np.float64 and tok.tolist() == [23.0]
+    assert logits.dtype == np.float32 and logits.shape == (1, 8) and (logits == 23.0).all()
+    assert FakeModel.built[-1].replays > 23
+    # above the size limit only the first sequences of the batch are kept
+    monkeypatch.setattr(bench, "DUMP_BYTES", 2 * 4 * 8)
+    bench.run_gpu(_args(no_extras=True, dump_outputs=str(out), batch=3), 0, 1, 0)
+    assert np.load(out / "next_token.npy").shape == (2,) and np.load(out / "logits.npy").shape == (2, 8)
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "x"]])
+def test_bench_rejects_arguments_it_cannot_honour(monkeypatch, argv):
+    import sys
+    monkeypatch.setattr(sys, "argv", ["bench.py"] + argv)
+    monkeypatch.setattr(bench, "run_gpu", lambda *a: pytest.fail("ran"))
+    monkeypatch.setattr(bench, "run_reference", lambda *a: pytest.fail("ran"))
+    with pytest.raises(SystemExit):
+        bench.main()
 
 
 def test_host_topology_and_the_reference_step(monkeypatch):
