@@ -1,5 +1,6 @@
-// Library-level plumbing: error string, ABI version, launch counter.
+// Library-level plumbing: error string, ABI version, launch counter, per-device launch settings.
 #include <stdarg.h>
+#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -15,6 +16,26 @@ void set_error(const char* fmt, ...) {
   va_start(ap, fmt);
   vsnprintf(g_err, sizeof(g_err), fmt, ap);
   va_end(ap);
+}
+
+int cur_device() {
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= kMaxDevices) dev = 0;
+  return dev;
+}
+
+int sm_count() {
+  static int n[kMaxDevices] = {};
+  const int dev = cur_device();
+  if (!n[dev]) {
+    if (cudaDeviceGetAttribute(&n[dev], cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n[dev] <= 0) n[dev] = kNumSMs;
+  }
+  return n[dev];
+}
+
+bool pdl_enabled() {
+  HQQ_ENV_KNOB(on, ([] { const char* e = getenv("HQQ_B200_PDL"); return (e && e[0] == '0') ? 0 : 1; })());
+  return on == 1;
 }
 
 }  // namespace hqq

@@ -49,6 +49,43 @@ static inline int64_t cdiv(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
 constexpr int kNumSMs = 148;  // B200
 
+// ---- kernel launches ------------------------------------------------------------------
+// Function attributes (opt-in dynamic shared memory) and SM counts belong to ONE device: the caches below are indexed by the
+// calling thread's current device, so layers living on several GPUs of one process each get their own setup.
+constexpr int kMaxDevices = 64;
+int cur_device();   // the calling thread's current device (0 if it cannot be told)
+int sm_count();     // SMs of the current device
+bool pdl_enabled(); // false under HQQ_B200_PDL=0 (test hook): the linear kernels launch without programmatic dependent launch
+
+// Raises kernel K's dynamic shared-memory limit on the current device to at least `bytes`.
+template <auto K>
+int reserve_smem(int bytes) {
+  static int have[kMaxDevices] = {};
+  int& h = have[cur_device()];
+  if (bytes > h) {
+    const cudaError_t e = cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    HQQ_REQUIRE(e == cudaSuccess, HQQ_E_CUDA, "hqq_b200_linear_fwd: cannot reserve %d bytes of shared memory: %s", bytes, cudaGetErrorString(e));
+    h = bytes;
+  }
+  return HQQ_OK;
+}
+
+// Counted launch, with the programmatic-stream-serialization attribute when `pdl` is set: the kernel may become resident
+// while its predecessor on the stream is still running, and waits for it in griddepcontrol.wait (pdl_wait).
+template <typename K, typename... Args>
+int launch_pdl(const char* name, K kernel, dim3 grid, dim3 block, size_t smem, cudaStream_t st, bool pdl, Args... args) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, args...);
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  HQQ_REQUIRE(e == cudaSuccess, HQQ_E_CUDA, "%s: CUDA launch failed: %s", name, cudaGetErrorString(e));
+  return HQQ_OK;
+}
+
 static inline int fields_of(int nbits) { return nbits == 3 ? 10 : 8 / nbits; }
 static inline bool valid_nbits(int nbits) { return nbits == 8 || nbits == 4 || nbits == 3 || nbits == 2 || nbits == 1; }
 static inline size_t dtype_size(int dt) {
@@ -66,6 +103,10 @@ template <typename T> __device__ __forceinline__ float to_f32(T v);
 template <> __device__ __forceinline__ float to_f32<float>(float v) { return v; }
 template <> __device__ __forceinline__ float to_f32<__half>(__half v) { return __half2float(v); }
 template <> __device__ __forceinline__ float to_f32<__nv_bfloat16>(__nv_bfloat16 v) { return __bfloat162float(v); }
+
+template <typename T> __device__ __forceinline__ T from_f32(float v);
+template <> __device__ __forceinline__ __half from_f32<__half>(float v) { return __float2half_rn(v); }
+template <> __device__ __forceinline__ __nv_bfloat16 from_f32<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
 
 // integer level -> T (levels are < 256: exact in every type)
 template <typename T> __device__ __forceinline__ T level_to(unsigned q);

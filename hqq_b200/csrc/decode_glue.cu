@@ -6,31 +6,9 @@
 #include <cooperative_groups.h>
 #endif
 
-#include "common.cuh"
+#include "device.cuh"
 
 namespace hqq {
-
-#ifdef HQQ_EMU
-// CPU emulation (tests/emu): kernels and blocks run one after another, so the dependency instructions, the L2 prefetch and the
-// system-scope accesses are plain code; the cluster argmax (DSMEM) is not emulated
-__device__ __forceinline__ void pdl_wait_g() {}
-__device__ __forceinline__ void pdl_launch_g() {}
-__device__ __forceinline__ uint32_t ld_sys_u32(const uint32_t* p) { return *reinterpret_cast<const volatile uint32_t*>(p); }
-__device__ __forceinline__ void prefetch_l2(const void*) {}
-#else
-__device__ __forceinline__ void pdl_wait_g() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_launch_g() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ uint32_t ld_sys_u32(const uint32_t* p) {
-  uint32_t v;
-  asm volatile("ld.relaxed.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
-#endif
-
-template <typename T> __device__ __forceinline__ T from_f32(float v);
-template <> __device__ __forceinline__ __half from_f32<__half>(float v) { return __float2half_rn(v); }
-template <> __device__ __forceinline__ __nv_bfloat16 from_f32<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
 
 __device__ __forceinline__ float block_sum(float v, float* red) {
 #pragma unroll
@@ -55,8 +33,8 @@ __global__ void __launch_bounds__(1024) add_rmsnorm_kernel(T* __restrict__ h, co
     y += row;
     if (delta) delta += row;
   }
-  pdl_launch_g();
-  pdl_wait_g();
+  pdl_launch_dependents();
+  pdl_wait();
   float v[8];
   int n = 0;
   float ss = 0.f;
@@ -82,8 +60,8 @@ template <typename T>
 __global__ void __launch_bounds__(1024) add_rmsnorm_tp_kernel(T* __restrict__ h, const uint32_t* red_data, int* step_ctr, int x_index, int x_per_step,
                                                               int tp, const T* __restrict__ w, T* __restrict__ y, int H, float eps) {
   __shared__ float red[32];
-  pdl_launch_g();
-  pdl_wait_g();
+  pdl_launch_dependents();
+  pdl_wait();
   const int step = *reinterpret_cast<volatile int*>(step_ctr);
   const uint32_t ex = (uint32_t)step * (uint32_t)x_per_step + (uint32_t)x_index;
   const uint32_t tag = ex & 0xFFFFu;
@@ -95,7 +73,7 @@ __global__ void __launch_bounds__(1024) add_rmsnorm_tp_kernel(T* __restrict__ h,
     float d = 0.f;
     for (int r = 0; r < tp; ++r) {
       uint32_t wv;
-      do { wv = ld_sys_u32(part + (size_t)r * H + i); } while ((wv >> 16) != tag);
+      do { wv = ld_relaxed_sys_u32(part + (size_t)r * H + i); } while ((wv >> 16) != tag);
       const unsigned short hb = (unsigned short)(wv & 0xFFFFu);
       d += to_f32<T>(*reinterpret_cast<const T*>(&hb));
     }
@@ -114,8 +92,8 @@ __global__ void __launch_bounds__(1024) add_rmsnorm_tp_kernel(T* __restrict__ h,
 // y = silu(g) * u
 template <typename T>
 __global__ void __launch_bounds__(256) silu_mul_kernel(const T* __restrict__ g, const T* __restrict__ u, T* __restrict__ y, int n) {
-  pdl_launch_g();
-  pdl_wait_g();
+  pdl_launch_dependents();
+  pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) {
     const float a = to_f32<T>(g[i]);
@@ -150,7 +128,7 @@ __global__ void __launch_bounds__(kAttnThreads) rope_attn_decode_kernel(const T*
     k_cache += b * n_kv * L * hd; v_cache += b * n_kv * L * hd;
   }
   const int pos = (int)pos_p[0];
-  pdl_launch_g();
+  pdl_launch_dependents();
   {
     // one 128-byte line per prefetch; pos rows of hd * sizeof(T) bytes each in both caches
     const char* kb = reinterpret_cast<const char*>(k_cache + (long long)kvh * L * hd);
@@ -161,7 +139,7 @@ __global__ void __launch_bounds__(kAttnThreads) rope_attn_decode_kernel(const T*
       prefetch_l2(vb + ((long long)i << 7));
     }
   }
-  pdl_wait_g();
+  pdl_wait();
   const int half = hd / 2;
   // rope: x*cos + rotate_half(x)*sin, computed in T like the framework ops
   if (d < hd) {
@@ -284,8 +262,8 @@ __global__ void __cluster_dims__(kArgmaxCtas, 1, 1) __launch_bounds__(1024) argm
   __shared__ unsigned long long xkey;
   cg::cluster_group cluster = cg::this_cluster();
   const int rank = (int)cluster.block_rank();
-  pdl_launch_g();
-  pdl_wait_g();
+  pdl_launch_dependents();
+  pdl_wait();
   float best = -INFINITY;
   int idx = 0;
   for (int i = (rank * 1024 + (int)threadIdx.x) * 8; i < n; i += kArgmaxCtas * 1024 * 8) {
@@ -354,20 +332,6 @@ __global__ void __cluster_dims__(kArgmaxCtas, 1, 1) __launch_bounds__(1024) argm
 
 #endif  // !HQQ_EMU
 
-template <typename K, typename... Args>
-static int launch_pdl(const char* name, K kernel, dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, args...);
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  HQQ_REQUIRE(e == cudaSuccess, HQQ_E_CUDA, "%s: CUDA launch failed: %s", name, cudaGetErrorString(e));
-  return HQQ_OK;
-}
-
 }  // namespace hqq
 
 using namespace hqq;
@@ -378,8 +342,8 @@ extern "C" int hqq_b200_glue_add_rmsnorm_rows(void* h, const void* delta, const 
               "hqq_b200_glue_add_rmsnorm: bad arguments (rows=%d H=%d)", rows, H);
   cudaStream_t st = (cudaStream_t)stream;
   const int threads = H > 2048 ? 1024 : 256;  // at most 8 elements per thread (the kernels keep them in registers)
-  if (dtype == HQQ_F16) return launch_pdl("add_rmsnorm", add_rmsnorm_kernel<__half>, dim3(rows), dim3(threads), 0, st, (__half*)h, (const __half*)delta, (const __half*)weight, (__half*)y, H, eps);
-  if (dtype == HQQ_BF16) return launch_pdl("add_rmsnorm", add_rmsnorm_kernel<__nv_bfloat16>, dim3(rows), dim3(threads), 0, st, (__nv_bfloat16*)h, (const __nv_bfloat16*)delta, (const __nv_bfloat16*)weight, (__nv_bfloat16*)y, H, eps);
+  if (dtype == HQQ_F16) return launch_pdl("add_rmsnorm", add_rmsnorm_kernel<__half>, dim3(rows), dim3(threads), 0, st, true, (__half*)h, (const __half*)delta, (const __half*)weight, (__half*)y, H, eps);
+  if (dtype == HQQ_BF16) return launch_pdl("add_rmsnorm", add_rmsnorm_kernel<__nv_bfloat16>, dim3(rows), dim3(threads), 0, st, true, (__nv_bfloat16*)h, (const __nv_bfloat16*)delta, (const __nv_bfloat16*)weight, (__nv_bfloat16*)y, H, eps);
   set_error("hqq_b200_glue_add_rmsnorm: dtype must be f16/bf16");
   return HQQ_E_INVALID;
 }
@@ -394,8 +358,8 @@ extern "C" int hqq_b200_glue_add_rmsnorm_tp(void* h, const void* red_data, int* 
               "hqq_b200_glue_add_rmsnorm_tp: bad arguments (H=%d tp=%d)", H, tp);
   cudaStream_t st = (cudaStream_t)stream;
   const int threads = H > 2048 ? 1024 : 256;  // at most 8 elements per thread (the kernels keep them in registers)
-  if (dtype == HQQ_F16) return launch_pdl("add_rmsnorm_tp", add_rmsnorm_tp_kernel<__half>, dim3(1), dim3(threads), 0, st, (__half*)h, (const uint32_t*)red_data, step_ctr, x_index, x_per_step, tp, (const __half*)weight, (__half*)y, H, eps);
-  if (dtype == HQQ_BF16) return launch_pdl("add_rmsnorm_tp", add_rmsnorm_tp_kernel<__nv_bfloat16>, dim3(1), dim3(threads), 0, st, (__nv_bfloat16*)h, (const uint32_t*)red_data, step_ctr, x_index, x_per_step, tp, (const __nv_bfloat16*)weight, (__nv_bfloat16*)y, H, eps);
+  if (dtype == HQQ_F16) return launch_pdl("add_rmsnorm_tp", add_rmsnorm_tp_kernel<__half>, dim3(1), dim3(threads), 0, st, true, (__half*)h, (const uint32_t*)red_data, step_ctr, x_index, x_per_step, tp, (const __half*)weight, (__half*)y, H, eps);
+  if (dtype == HQQ_BF16) return launch_pdl("add_rmsnorm_tp", add_rmsnorm_tp_kernel<__nv_bfloat16>, dim3(1), dim3(threads), 0, st, true, (__nv_bfloat16*)h, (const uint32_t*)red_data, step_ctr, x_index, x_per_step, tp, (const __nv_bfloat16*)weight, (__nv_bfloat16*)y, H, eps);
   set_error("hqq_b200_glue_add_rmsnorm_tp: dtype must be f16/bf16");
   return HQQ_E_INVALID;
 }
@@ -404,8 +368,8 @@ extern "C" int hqq_b200_glue_silu_mul(const void* gate, const void* up, void* y,
   HQQ_REQUIRE(gate && up && y && n > 0, HQQ_E_INVALID, "hqq_b200_glue_silu_mul: bad arguments");
   cudaStream_t st = (cudaStream_t)stream;
   const dim3 grid((unsigned)cdiv(n, 256));
-  if (dtype == HQQ_F16) return launch_pdl("silu_mul", silu_mul_kernel<__half>, grid, dim3(256), 0, st, (const __half*)gate, (const __half*)up, (__half*)y, n);
-  if (dtype == HQQ_BF16) return launch_pdl("silu_mul", silu_mul_kernel<__nv_bfloat16>, grid, dim3(256), 0, st, (const __nv_bfloat16*)gate, (const __nv_bfloat16*)up, (__nv_bfloat16*)y, n);
+  if (dtype == HQQ_F16) return launch_pdl("silu_mul", silu_mul_kernel<__half>, grid, dim3(256), 0, st, true, (const __half*)gate, (const __half*)up, (__half*)y, n);
+  if (dtype == HQQ_BF16) return launch_pdl("silu_mul", silu_mul_kernel<__nv_bfloat16>, grid, dim3(256), 0, st, true, (const __nv_bfloat16*)gate, (const __nv_bfloat16*)up, (__nv_bfloat16*)y, n);
   set_error("hqq_b200_glue_silu_mul: dtype must be f16/bf16");
   return HQQ_E_INVALID;
 }
@@ -423,7 +387,7 @@ extern "C" int hqq_b200_glue_rope_attn_decode_batch(const void* q, const void* k
   const float scale = 1.0f / sqrtf((float)head_dim);
   auto go = [&](auto kernel, auto tag) {
     using T = decltype(tag);
-    return launch_pdl("rope_attn_decode", kernel, dim3(n_q_heads, batch), dim3(kAttnThreads), smem, st, (const T*)q, (const T*)k, (const T*)v,
+    return launch_pdl("rope_attn_decode", kernel, dim3(n_q_heads, batch), dim3(kAttnThreads), smem, st, true, (const T*)q, (const T*)k, (const T*)v,
                       (const T*)cos_table, (const T*)sin_table, (T*)k_cache, (T*)v_cache, (const long long*)pos, (T*)out, n_q_heads, n_kv_heads,
                       cache_len, head_dim, scale);
   };
@@ -446,8 +410,8 @@ extern "C" int hqq_b200_glue_rope_attn_decode(const void* q, const void* k, cons
 extern "C" int hqq_b200_glue_argmax(const void* logits, int n, int64_t* out, int dtype, void* stream) {
   HQQ_REQUIRE(logits && out && n > 0, HQQ_E_INVALID, "hqq_b200_glue_argmax: bad arguments");
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == HQQ_F16) return launch_pdl("argmax", argmax_kernel<__half>, dim3(kArgmaxCtas), dim3(1024), 0, st, (const __half*)logits, n, (long long*)out, -1LL, KeyPeers{}, 0, 0, (const int*)nullptr);
-  if (dtype == HQQ_BF16) return launch_pdl("argmax", argmax_kernel<__nv_bfloat16>, dim3(kArgmaxCtas), dim3(1024), 0, st, (const __nv_bfloat16*)logits, n, (long long*)out, -1LL, KeyPeers{}, 0, 0, (const int*)nullptr);
+  if (dtype == HQQ_F16) return launch_pdl("argmax", argmax_kernel<__half>, dim3(kArgmaxCtas), dim3(1024), 0, st, true, (const __half*)logits, n, (long long*)out, -1LL, KeyPeers{}, 0, 0, (const int*)nullptr);
+  if (dtype == HQQ_BF16) return launch_pdl("argmax", argmax_kernel<__nv_bfloat16>, dim3(kArgmaxCtas), dim3(1024), 0, st, true, (const __nv_bfloat16*)logits, n, (long long*)out, -1LL, KeyPeers{}, 0, 0, (const int*)nullptr);
   set_error("hqq_b200_glue_argmax: dtype must be f16/bf16");
   return HQQ_E_INVALID;
 }
@@ -455,8 +419,8 @@ extern "C" int hqq_b200_glue_argmax(const void* logits, int n, int64_t* out, int
 extern "C" int hqq_b200_glue_argmax_key(const void* logits, int n, int64_t index_offset, int64_t* out_key, int dtype, void* stream) {
   HQQ_REQUIRE(logits && out_key && n > 0 && index_offset >= 0 && index_offset + n <= 0xFFFFFFFFll, HQQ_E_INVALID, "hqq_b200_glue_argmax_key: bad arguments");
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == HQQ_F16) return launch_pdl("argmax_key", argmax_kernel<__half>, dim3(kArgmaxCtas), dim3(1024), 0, st, (const __half*)logits, n, (long long*)out_key, (long long)index_offset, KeyPeers{}, 0, 0, (const int*)nullptr);
-  if (dtype == HQQ_BF16) return launch_pdl("argmax_key", argmax_kernel<__nv_bfloat16>, dim3(kArgmaxCtas), dim3(1024), 0, st, (const __nv_bfloat16*)logits, n, (long long*)out_key, (long long)index_offset, KeyPeers{}, 0, 0, (const int*)nullptr);
+  if (dtype == HQQ_F16) return launch_pdl("argmax_key", argmax_kernel<__half>, dim3(kArgmaxCtas), dim3(1024), 0, st, true, (const __half*)logits, n, (long long*)out_key, (long long)index_offset, KeyPeers{}, 0, 0, (const int*)nullptr);
+  if (dtype == HQQ_BF16) return launch_pdl("argmax_key", argmax_kernel<__nv_bfloat16>, dim3(kArgmaxCtas), dim3(1024), 0, st, true, (const __nv_bfloat16*)logits, n, (long long*)out_key, (long long)index_offset, KeyPeers{}, 0, 0, (const int*)nullptr);
   set_error("hqq_b200_glue_argmax_key: dtype must be f16/bf16");
   return HQQ_E_INVALID;
 }
@@ -472,8 +436,8 @@ extern "C" int hqq_b200_glue_argmax_tp(const void* logits, int n, int64_t index_
     kp.p[i] = (unsigned long long*)peer_keys[i];
   }
   cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == HQQ_F16) return launch_pdl("argmax_tp", argmax_kernel<__half>, dim3(kArgmaxCtas), dim3(1024), 0, st, (const __half*)logits, n, (long long*)out, (long long)index_offset, kp, tp, rank, step_ctr);
-  if (dtype == HQQ_BF16) return launch_pdl("argmax_tp", argmax_kernel<__nv_bfloat16>, dim3(kArgmaxCtas), dim3(1024), 0, st, (const __nv_bfloat16*)logits, n, (long long*)out, (long long)index_offset, kp, tp, rank, step_ctr);
+  if (dtype == HQQ_F16) return launch_pdl("argmax_tp", argmax_kernel<__half>, dim3(kArgmaxCtas), dim3(1024), 0, st, true, (const __half*)logits, n, (long long*)out, (long long)index_offset, kp, tp, rank, step_ctr);
+  if (dtype == HQQ_BF16) return launch_pdl("argmax_tp", argmax_kernel<__nv_bfloat16>, dim3(kArgmaxCtas), dim3(1024), 0, st, true, (const __nv_bfloat16*)logits, n, (long long*)out, (long long)index_offset, kp, tp, rank, step_ctr);
   set_error("hqq_b200_glue_argmax_tp: dtype must be f16/bf16");
   return HQQ_E_INVALID;
 }

@@ -22,7 +22,7 @@
 #include <stdlib.h>
 #include <cuda.h>  // CUtensorMap types only; the encode entry point is resolved through the runtime (no -lcuda)
 
-#include "common.cuh"
+#include "device.cuh"
 
 namespace hqq {
 
@@ -90,15 +90,6 @@ __host__ __device__ __forceinline__ Item decode_item(const Args& a, int j) {
   return it;
 }
 
-// programmatic dependent launch: the split-K second pass is a dependent of the GEMM grid
-#ifdef HQQ_EMU
-__device__ __forceinline__ void pdl_wait_primary() {}
-__device__ __forceinline__ void pdl_release_dependents() {}
-#else
-__device__ __forceinline__ void pdl_wait_primary() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_release_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-#endif
-
 // ---- PTX wrappers -------------------------------------------------------------------------------------------------
 #ifdef HQQ_EMU
 // CPU emulation (tests/emu): the same entry points, backed by a functional model of mbarrier / TMA / tcgen05 / TMEM
@@ -122,7 +113,6 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) { :
 #define HQQ_STS_V4(addr, a, b, c, d) ::emu::sts(addr, a, b, c, d)
 #define HQQ_STS_V2(addr, a, b) ::emu::sts(addr, a, b)
 #define HQQ_PREFETCH_TENSORMAP(p) ((void)(p))
-#define HQQ_PREFETCH_L2(p) ((void)(p))
 #define HQQ_NAMED_BAR_SYNC(id, n) ::emu::named_barrier(id, n)
 #else
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -196,7 +186,6 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
 #define HQQ_STS_V4(addr, a, b, c, d) asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory")
 #define HQQ_STS_V2(addr, a, b) asm volatile("st.shared.v2.b32 [%0], {%1,%2};" ::"r"(addr), "r"(a), "r"(b) : "memory")
 #define HQQ_PREFETCH_TENSORMAP(p) asm volatile("prefetch.tensormap [%0];" ::"l"(p) : "memory")
-#define HQQ_PREFETCH_L2(p) asm volatile("prefetch.global.L2 [%0];" ::"l"(p))
 #define HQQ_NAMED_BAR_SYNC(id, n) asm volatile("bar.sync %0, %1;" ::"n"(id), "n"(n) : "memory")
 #endif  // HQQ_EMU
 
@@ -227,17 +216,6 @@ __device__ __forceinline__ uint32_t make_idesc(int UN) {
 }
 
 // ---- level -> T with the reference's roundings -------------------------------------------------------------------
-// Two k-adjacent levels (bytes b0, b1 already masked to the field) -> T2 {fl(fl(q0 - z) * s), fl(fl(q1 - z) * s)}.
-__device__ __forceinline__ uint32_t prmt_b32(uint32_t a, uint32_t b, uint32_t sel) {
-#ifdef HQQ_EMU
-  return ::emu::prmt(a, b, sel);
-#else
-  uint32_t r;
-  asm("prmt.b32 %0, %1, %2, %3;" : "=r"(r) : "r"(a), "r"(b), "r"(sel));
-  return r;
-#endif
-}
-
 // Four k-adjacent levels (one per byte of `t`, already masked to the field) -> two packed T2
 //   {fl(fl(q0 - z) * s), fl(fl(q1 - z) * s)}, {.. q2, q3 ..}
 template <typename T> struct Pair;
@@ -247,7 +225,7 @@ template <> struct Pair<__half> {
     // byte | 0x6400 == 1024 + q exactly (one PRMT per pair); subtracting 1024 is exact, so (q - z) and (.. * s) round
     // exactly like the reference's two steps
     const __half2 k1024 = __half2half2(__ushort_as_half((unsigned short)0x6400));
-    uint32_t a = prmt_b32(t, 0x64646464u, 0x4140u), b = prmt_b32(t, 0x64646464u, 0x4342u);
+    uint32_t a = prmt(t, 0x64646464u, 0x4140u), b = prmt(t, 0x64646464u, 0x4342u);
     __half2 ha = __hmul2(__hsub2(__hsub2(*reinterpret_cast<__half2*>(&a), k1024), z2), s2);
     __half2 hb = __hmul2(__hsub2(__hsub2(*reinterpret_cast<__half2*>(&b), k1024), z2), s2);
     lo = *reinterpret_cast<uint32_t*>(&ha);
@@ -268,10 +246,6 @@ template <> struct Pair<__nv_bfloat16> {
   }
   __device__ __forceinline__ static __nv_bfloat162 bcast(__nv_bfloat16 v) { return __bfloat162bfloat162(v); }
 };
-
-template <typename T> __device__ __forceinline__ T cvt_out(float v);
-template <> __device__ __forceinline__ __half cvt_out<__half>(float v) { return __float2half_rn(v); }
-template <> __device__ __forceinline__ __nv_bfloat16 cvt_out<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
 
 
 struct Smem {
@@ -335,13 +309,13 @@ __global__ void __launch_bounds__(kThreads, 1) linear_gemm_kernel(const __grid_c
   // predecessor may still be writing is the activation x (and, dense mode, W written by the dequantize kernel): the TMA producer
   // waits before its first load, and nothing is written (y, split-K partials) before an accumulator fed by those loads is full.
   // Packed weights, scale, zero and bias are never produced by a kernel that releases its dependents early.
-  if (threadIdx.x == 0) pdl_release_dependents();
+  if (threadIdx.x == 0) pdl_launch_dependents();
 
   if (warp == 0) {
     // ================= TMA producer: activation tiles =================
     if (lane == 0) {
       uint32_t it = 0;  // k-blocks issued so far (ring position)
-      pdl_wait_primary();
+      pdl_wait();
       for (int j = blockIdx.x; j < n_items; j += gridDim.x) {
         const Item im = decode_item(a, j);
         if (!im.valid) continue;
@@ -465,7 +439,7 @@ __global__ void __launch_bounds__(kThreads, 1) linear_gemm_kernel(const __grid_c
           // the register prefetch reaches one quad ahead, about 1 us of main loop at small M -- less than a DRAM round trip under
           // load when a weight tile is read for the first time (M <= 512: every tile is); pull the line this thread will load
           // three quads from now into L2 (a packed row has 256 bytes = two lines per quad: even / odd threads of the row take one each)
-          if (q + 4 < num_quads) HQQ_PREFETCH_L2(wptr + 3 * 4 * kBlockK + (c & 1) * 128);
+          if (q + 4 < num_quads) prefetch_l2(wptr + 3 * 4 * kBlockK + (c & 1) * 128);
           load_quad();
         } else if (jn < n_items) {
           tile_ptrs(decode_item(a, jn));
@@ -520,7 +494,7 @@ __global__ void __launch_bounds__(kThreads, 1) linear_gemm_kernel(const __grid_c
       const int prow0 = im.tile_n * PR;
       const bool n_ok = (prow0 + tp) < a.step;
       const int n = tf * a.step + prow0 + tp;
-      T bn = cvt_out<T>(0.0f);
+      T bn = from_f32<T>(0.0f);
       if (has_bias && n_ok) bn = bias[n];
       mbar_wait(&acc_full[buf], use & 1);
       tc_fence_after();
@@ -539,7 +513,7 @@ __global__ void __launch_bounds__(kThreads, 1) linear_gemm_kernel(const __grid_c
           for (int jj = 0; jj < 32; ++jj) {
             const int m = im.m0 + col + jj;
             if (n_ok && m < a.M) {
-              T o = cvt_out<T>(__uint_as_float(v[jj]));
+              T o = from_f32<T>(__uint_as_float(v[jj]));
               if (has_bias) o = __hadd(o, bn);  // out += bias: second rounding, as in the reference
               y[(long long)m * a.N + n] = o;
             }
@@ -567,7 +541,7 @@ template <typename T, int V>
 __global__ void __launch_bounds__(256) splitk_reduce_kernel(const float* __restrict__ ws, T* __restrict__ y, const T* __restrict__ bias, int M, int N,
                                                             int step, int PR, int S, int n_row, int n_tok) {
   const long long idx = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * V;
-  pdl_wait_primary();  // launched as a programmatic dependent of the GEMM: resident early, reads only after that grid has completed
+  pdl_wait();  // launched as a programmatic dependent of the GEMM: resident early, reads only after that grid has completed
   if (idx >= (long long)M * N) return;
   const int m = (int)(idx / N), n = (int)(idx % N);
   const int f = n / step, prg = n % step;
@@ -596,7 +570,7 @@ __global__ void __launch_bounds__(256) splitk_reduce_kernel(const float* __restr
 #pragma unroll
     for (int sidx = 0; sidx < 8; ++sidx)
       if (sidx < S) acc += part[sidx][v];
-    o[v] = cvt_out<T>(acc);
+    o[v] = from_f32<T>(acc);
     if (bias) o[v] = __hadd(o[v], bias[n + v]);
   }
   if constexpr (V == 4) {
@@ -639,12 +613,6 @@ static int encode_map(CUtensorMap* xmap, const void* x, int64_t rows, int64_t K,
   return HQQ_OK;
 }
 
-static int sm_count() {
-  int dev = 0, n = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = kNumSMs;
-  return n;
-}
-
 // see `Sched`: full tiles first, the last partial round as half tiles when that shortens it
 // HQQ_B200_GEMM_CTAS=<n> (test hook): the number of persistent CTAs the schedule is built for instead of the SM count, so that
 // small problems exercise tile-after-tile execution, both accumulators, the half-tile round and split-K (the emulator tests and
@@ -652,12 +620,6 @@ static int sm_count() {
 static int persistent_ctas() {
   HQQ_ENV_KNOB(cta_cap, ([] { const char* e = getenv("HQQ_B200_GEMM_CTAS"); return e ? atoi(e) : 0; })());
   return cta_cap > 0 ? cta_cap : sm_count();
-}
-
-// HQQ_B200_PDL=0 (test hook, shared with the small-M kernels): launch without the programmatic-dependency attribute
-static bool pdl_on() {
-  HQQ_ENV_KNOB(on, ([] { const char* e = getenv("HQQ_B200_PDL"); return (e && e[0] == '0') ? 0 : 1; })());
-  return on == 1;
 }
 
 // HQQ_B200_GEMM_KSPLIT=<n> (test / measurement hook): the largest number of k-slices the schedule may use (1 = never split)
@@ -721,47 +683,18 @@ static int launch(const void* x, Args& a, cudaStream_t st, const void* dense_W =
     a.ws = reinterpret_cast<float*>(ws);
   }
   const int grid = a.sched.n_items < P ? a.sched.n_items : P;
-  auto k = linear_gemm_kernel<T, NBITS, GS>;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  static bool attr_set[64] = {};  // per device: the attribute belongs to the function on ONE device
-  if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem::BYTES);
-    HQQ_REQUIRE(e == cudaSuccess, HQQ_E_CUDA, "hqq_b200_linear_fwd: cannot reserve %d bytes of shared memory: %s", Smem::BYTES, cudaGetErrorString(e));
-    if (dev >= 0 && dev < 64) attr_set[dev] = true;
-  }
-  {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = Smem::BYTES;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl_on() ? 1 : 0;
-    cudaLaunchKernelEx(&cfg, k, xmap256, xmap128, amap, a);
-  }
-  HQQ_LAUNCH_CHECK("hqq_b200_linear_fwd/tcgen05");
+  constexpr auto k = linear_gemm_kernel<T, NBITS, GS>;
+  rc = reserve_smem<k>(Smem::BYTES);
+  if (rc) return rc;
+  rc = launch_pdl("hqq_b200_linear_fwd/tcgen05", k, dim3((unsigned)grid), dim3(kThreads), Smem::BYTES, st, pdl_enabled(), xmap256, xmap128, amap, a);
+  if (rc) return rc;
   if (a.sched.ksplit > 1) {
     const long long total = (long long)a.M * a.N;
     const bool vec = a.step % 4 == 0 && PR % 4 == 0 && aligned(a.y, 8);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)cdiv(vec ? total / 4 : total, 256));
-    cfg.blockDim = dim3(256);
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl_on() ? 1 : 0;
-    T* yt = reinterpret_cast<T*>(a.y);
-    const T* bt = reinterpret_cast<const T*>(a.bias);
-    const float* wsc = a.ws;
-    if (vec) cudaLaunchKernelEx(&cfg, splitk_reduce_kernel<T, 4>, wsc, yt, bt, a.M, a.N, a.step, (int)PR, a.sched.ksplit, a.sched.n_row, a.sched.n_tok);
-    else cudaLaunchKernelEx(&cfg, splitk_reduce_kernel<T, 1>, wsc, yt, bt, a.M, a.N, a.step, (int)PR, a.sched.ksplit, a.sched.n_row, a.sched.n_tok);
-    HQQ_LAUNCH_CHECK("hqq_b200_linear_fwd/splitk-reduce");
+    const auto reduce = vec ? splitk_reduce_kernel<T, 4> : splitk_reduce_kernel<T, 1>;
+    return launch_pdl("hqq_b200_linear_fwd/splitk-reduce", reduce, dim3((unsigned)cdiv(vec ? total / 4 : total, 256)), dim3(256), 0, st, pdl_enabled(),
+                      (const float*)a.ws, reinterpret_cast<T*>(a.y), reinterpret_cast<const T*>(a.bias), a.M, a.N, a.step, (int)PR, a.sched.ksplit,
+                      a.sched.n_row, a.sched.n_tok);
   }
   return HQQ_OK;
 }

@@ -20,9 +20,9 @@
 // memory in a fixed order: deterministic, no atomics, no workspace.  Launched with programmatic dependent launch: the
 // weight prefetch starts before the producer of x has finished.
 #include <stdlib.h>
-#include <string.h>
 #include <type_traits>
 
+#include "device.cuh"
 #include "linear_internal.cuh"
 
 namespace hqq {
@@ -82,117 +82,36 @@ struct SKArgs {
   int x_index, x_per_step;
 };
 
-#ifdef HQQ_EMU
-#define HQQ_ST_RELAXED_SYS(p, v) (*reinterpret_cast<volatile uint32_t*>(p) = (v))
-#else
-#define HQQ_ST_RELAXED_SYS(p, v) asm volatile("st.relaxed.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory")
-#endif
-
-template <typename T> struct MT16;
-template <> struct MT16<__half> {
-  static constexpr uint32_t ONE2 = 0x3C003C00u;
-  __device__ __forceinline__ static void mma(float (&d)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
-#ifndef HQQ_EMU
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-                 : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-#else
-    ::emu::mma_m16n8k16<__half>(d, a0, a1, a2, a3, b0, b1, false);
-#endif
-  }
-  // same with C = 0 (first MMA of a group): no accumulator clearing instructions needed
-  __device__ __forceinline__ static void mma0(float (&d)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
-#ifndef HQQ_EMU
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%10,%10,%10,%10};"
-                 : "=f"(d[0]), "=f"(d[1]), "=f"(d[2]), "=f"(d[3])
-                 : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1), "f"(0.0f));
-#else
-    ::emu::mma_m16n8k16<__half>(d, a0, a1, a2, a3, b0, b1, true);
-#endif
-  }
-  __device__ __forceinline__ static float ld(const void* p, long long i) { return __half2float(reinterpret_cast<const __half*>(p)[i]); }
-  __device__ __forceinline__ static __half cvt(float v, const void* bias, int n) {
-    __half o = __float2half_rn(v);
-    if (bias) o = __hadd(o, reinterpret_cast<const __half*>(bias)[n]);  // out += bias, second rounding as in the reference
+// the 16-bit activation / output type of an MMA tile
+template <typename T> struct MT16 {
+  static constexpr uint32_t ONE2 = std::is_same<T, __half>::value ? 0x3C003C00u : 0x3F803F80u;  // {1, 1}: the all-ones A tile
+  __device__ __forceinline__ static T cvt(float v, const void* bias, int n) {
+    T o = from_f32<T>(v);
+    if (bias) o = __hadd(o, reinterpret_cast<const T*>(bias)[n]);  // out += bias, second rounding as in the reference
     return o;
   }
-  __device__ __forceinline__ static void st(void* p, long long i, float v, const void* bias, int n) { reinterpret_cast<__half*>(p)[i] = cvt(v, bias, n); }
-};
-template <> struct MT16<__nv_bfloat16> {
-  static constexpr uint32_t ONE2 = 0x3F803F80u;
-  __device__ __forceinline__ static void mma(float (&d)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
-#ifndef HQQ_EMU
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-                 : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-#else
-    ::emu::mma_m16n8k16<__nv_bfloat16>(d, a0, a1, a2, a3, b0, b1, false);
-#endif
-  }
-  __device__ __forceinline__ static void mma0(float (&d)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
-#ifndef HQQ_EMU
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%10,%10,%10,%10};"
-                 : "=f"(d[0]), "=f"(d[1]), "=f"(d[2]), "=f"(d[3])
-                 : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1), "f"(0.0f));
-#else
-    ::emu::mma_m16n8k16<__nv_bfloat16>(d, a0, a1, a2, a3, b0, b1, true);
-#endif
-  }
-  __device__ __forceinline__ static float ld(const void* p, long long i) { return __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(p)[i]); }
-  __device__ __forceinline__ static __nv_bfloat16 cvt(float v, const void* bias, int n) {
-    __nv_bfloat16 o = __float2bfloat16_rn(v);
-    if (bias) o = __hadd(o, reinterpret_cast<const __nv_bfloat16*>(bias)[n]);
-    return o;
-  }
-  __device__ __forceinline__ static void st(void* p, long long i, float v, const void* bias, int n) { reinterpret_cast<__nv_bfloat16*>(p)[i] = cvt(v, bias, n); }
+  __device__ __forceinline__ static void st(void* p, long long i, float v, const void* bias, int n) { reinterpret_cast<T*>(p)[i] = cvt(v, bias, n); }
 };
 
-__device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b, uint32_t s) {
-#ifdef HQQ_EMU
-  return ::emu::prmt(a, b, s);
-#else
-  uint32_t r;
-  asm("prmt.b32 %0, %1, %2, %3;" : "=r"(r) : "r"(a), "r"(b), "r"(s));
-  return r;
-#endif
-}
-template <int LUT>
-__device__ __forceinline__ uint32_t lop3(uint32_t a, uint32_t b, uint32_t c) {
-#ifdef HQQ_EMU
-  return ::emu::lop3(a, b, c, (uint32_t)LUT);
-#else
-  uint32_t r;
-  asm("lop3.b32 %0, %1, %2, %3, %4;" : "=r"(r) : "r"(a), "r"(b), "r"(c), "n"(LUT));
-  return r;
-#endif
-}
 // (a & b) | c
 __device__ __forceinline__ uint32_t and_or(uint32_t a, uint32_t b, uint32_t c) { return lop3<0xEA>(a, b, c); }
 
 // How the integer levels are planted into 16-bit float lanes (lane value = OFF + q * V):
-//   MAGIC_OFFSET    fp16: bits | 0x6400 -> 1024 + q*2^sh          bf16: (bits >> sh) | 0x4300 -> 128 + q
-//   MAGIC_SUBNORMAL fp16 only: bits taken as a subnormal          -> q * 2^(sh-24)   (no offset, exact)
-enum { MAGIC_OFFSET = 0, MAGIC_SUBNORMAL = 1 };
-
-template <typename T, int NBITS, int MAGIC> struct Lanes;
+//   fp16: bits | 0x6400 -> 1024 + q*2^sh          bf16: (bits >> sh) | 0x4300 -> 128 + q
+template <typename T, int NBITS> struct Lanes;
 
 // fp16, sub-byte fields: mask in place, no shift (1 PRMT + 1 SHF + 4 LOP3 per 8 weights)
-template <int NBITS, int MAGIC>
-struct Lanes<__half, NBITS, MAGIC> {
-  static constexpr uint32_t OR = (MAGIC == MAGIC_OFFSET) ? 0x64006400u : 0u;
+template <int NBITS>
+struct Lanes<__half, NBITS> {
+  static constexpr uint32_t OR = 0x64006400u;
   uint32_t mask_a, mask_b;
   float invV_a, invV_b, offV_a, offV_b;
   __device__ __forceinline__ void init(int sh_a, int sh_b) {
     const uint32_t m = (1u << NBITS) - 1u;
     mask_a = (m << sh_a) * 0x00010001u;
     mask_b = (m << sh_b) * 0x00010001u;
-    if (MAGIC == MAGIC_OFFSET) {
-      invV_a = exp2f(-(float)sh_a); invV_b = exp2f(-(float)sh_b);
-      offV_a = 1024.0f * invV_a;    offV_b = 1024.0f * invV_b;
-    } else {
-      invV_a = exp2f(24.0f - (float)sh_a); invV_b = exp2f(24.0f - (float)sh_b);
-      offV_a = 0.0f; offV_b = 0.0f;
-    }
+    invV_a = exp2f(-(float)sh_a); invV_b = exp2f(-(float)sh_b);
+    offV_a = 1024.0f * invV_a;    offV_b = 1024.0f * invV_b;
   }
   // w: 4 consecutive k-bytes of one packed row.  a0/a2: field A for k{0,1} / k{2,3}; a1/a3: field B.
   __device__ __forceinline__ void extract(uint32_t w, uint32_t& a0, uint32_t& a1, uint32_t& a2, uint32_t& a3) const {
@@ -214,8 +133,8 @@ struct Lanes<__half, NBITS, MAGIC> {
 };
 
 // bf16, sub-byte fields: only 7 mantissa bits -> shift the field down to bit 0 first
-template <int NBITS, int MAGIC>
-struct Lanes<__nv_bfloat16, NBITS, MAGIC> {
+template <int NBITS>
+struct Lanes<__nv_bfloat16, NBITS> {
   int sh_a, sh_b;
   float invV_a, invV_b, offV_a, offV_b;
   __device__ __forceinline__ void init(int sa, int sb) {
@@ -241,14 +160,11 @@ struct Lanes<__nv_bfloat16, NBITS, MAGIC> {
 };
 
 // fp16, 8-bit: whole bytes, two packed rows per thread (rows r and r+8 of the tile)
-template <int MAGIC>
-struct Lanes<__half, 8, MAGIC> {
-  static constexpr uint32_t HB = (MAGIC == MAGIC_OFFSET) ? 0x64646464u : 0u;
+template <>
+struct Lanes<__half, 8> {
+  static constexpr uint32_t HB = 0x64646464u;
   float invV_a, invV_b, offV_a, offV_b;
-  __device__ __forceinline__ void init(int, int) {
-    if (MAGIC == MAGIC_OFFSET) { invV_a = invV_b = 1.0f; offV_a = offV_b = 1024.0f; }
-    else { invV_a = invV_b = 16777216.0f; offV_a = offV_b = 0.0f; }
-  }
+  __device__ __forceinline__ void init(int, int) { invV_a = invV_b = 1.0f; offV_a = offV_b = 1024.0f; }
   __device__ __forceinline__ void extract2(uint32_t wa, uint32_t wb, uint32_t& a0, uint32_t& a1, uint32_t& a2, uint32_t& a3) const {
     a0 = prmt(wa, HB, 0x4140u);  // lanes {k0, k1} of row r
     a2 = prmt(wa, HB, 0x4342u);  // lanes {k2, k3}
@@ -263,73 +179,17 @@ struct Lanes<__half, 8, MAGIC> {
   }
 };
 
-__device__ __forceinline__ void cp_async16(void* smem, const void* g) {
-#ifdef HQQ_EMU
-  ::emu::cp_async(smem, g, 16);  // lands at the wait_group that covers it (tests/emu)
-#else
-  const uint32_t s = (uint32_t)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s), "l"(g) : "memory");
-#endif
-}
-template <int BYTES>
-__device__ __forceinline__ void cp_async_small(void* smem, const void* g) {
-#ifdef HQQ_EMU
-  ::emu::cp_async(smem, g, BYTES);
-#else
-  const uint32_t s = (uint32_t)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.ca.shared.global [%0], [%1], %2;" ::"r"(s), "l"(g), "n"(BYTES) : "memory");
-#endif
-}
-#ifdef HQQ_EMU
-__device__ __forceinline__ void cp_async_commit() { ::emu::cp_async_commit(); }
-template <int N> __device__ __forceinline__ void cp_async_wait() { ::emu::cp_async_wait(N); }
-__device__ __forceinline__ void pdl_wait() {}
-__device__ __forceinline__ void pdl_launch_dependents() {}
-#else
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-#endif
-
-template <typename T> __device__ __forceinline__ T from_f32_t(float v);
-template <> __device__ __forceinline__ __half from_f32_t<__half>(float v) { return __float2half_rn(v); }
-template <> __device__ __forceinline__ __nv_bfloat16 from_f32_t<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
-
-__device__ __forceinline__ int ld_acquire_sys(const int* p) {
-#ifdef HQQ_EMU
-  return *reinterpret_cast<const volatile int*>(p);
-#else
-  int v;
-  asm volatile("ld.acquire.sys.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-#endif
-}
-__device__ __forceinline__ void st_release_sys(int* p, int v) {
-#ifdef HQQ_EMU
-  *reinterpret_cast<volatile int*>(p) = v;
-#else
-  asm volatile("st.release.sys.global.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-#endif
-}
-
-#ifndef HQQ_EMU
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-#endif
-
-template <typename T, int NBITS, int GS, int MT, int MAGIC>
+template <typename T, int NBITS, int GS, int MT>
 struct SKCfg {
   static constexpr int F = 8 / NBITS;            // fields (slabs) per byte
   static constexpr int P = 16 / F;               // packed rows per 16-row MMA tile
   static constexpr int MPG = GS / 16;            // MMAs per quantisation group
   static constexpr int GPB = 256 / GS;           // quantisation groups per 256-k unit
-  static constexpr int MB = GPB * 2;             // bytes of scale (or zero) per unit and row
   static constexpr int NWV = (F == 1) ? 8 : 4;   // 16-byte weight vectors per thread and unit
   static constexpr int ST = (F == 1) ? 2 : 4;    // ring stages
-  static constexpr int W_BYTES = ST * NWV * 256 * 16;
-  static constexpr int M_BYTES = 0;                     // scale/zero travel through registers
+  static constexpr int W_BYTES = ST * NWV * 256 * 16;   // scale/zero travel through registers
   static constexpr int P_BYTES = 2 * 8 * MT * 128 * 4;  // double-buffered split-K partials, one 16x8 tile per warp
-  static constexpr int SMEM = W_BYTES + M_BYTES + P_BYTES;
+  static constexpr int SMEM = W_BYTES + P_BYTES;
   static constexpr int MIN_CTAS = (SMEM <= 110 * 1024 && MT <= 2) ? 2 : 1;
 };
 
@@ -338,20 +198,20 @@ struct SKCfg {
 // per-thread cp.async rings (the ring keeps prefetching across tile boundaries, so HBM requests never drain).  Partials
 // meet in shared memory once per tile (one block barrier, double-buffered) and warp (tile % 8) adds them in warp order:
 // deterministic, no atomics, no global workspace.
-template <typename T, int NBITS, int GS, int MT, int MAGIC>
-__global__ void __launch_bounds__(256, SKCfg<T, NBITS, GS, MT, MAGIC>::MIN_CTAS) linear_small_kernel(const __grid_constant__ SKArgs a) {
-  using C = SKCfg<T, NBITS, GS, MT, MAGIC>;
+template <typename T, int NBITS, int GS, int MT>
+__global__ void __launch_bounds__(256, SKCfg<T, NBITS, GS, MT>::MIN_CTAS) linear_small_kernel(const __grid_constant__ SKArgs a) {
+  using C = SKCfg<T, NBITS, GS, MT>;
   constexpr int F = C::F, P = C::P, MPG = C::MPG, GPB = C::GPB, NWV = C::NWV, ST = C::ST;
   using MM = MT16<T>;
   extern __shared__ __align__(16) uint8_t smem[];
-  uint4* wring = reinterpret_cast<uint4*>(smem);                             // [ST][NWV][256] one 16-byte slot per thread
-  float* part_s = reinterpret_cast<float*>(smem + C::W_BYTES + C::M_BYTES);  // [2][8][MT][128]
+  uint4* wring = reinterpret_cast<uint4*>(smem);                  // [ST][NWV][256] one 16-byte slot per thread
+  float* part_s = reinterpret_cast<float*>(smem + C::W_BYTES);  // [2][8][MT][128]
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int r = lane >> 2, c = lane & 3;
   const int p = (F == 1) ? r : (r % P);
   const int fa = (F == 1) ? 0 : (r / P), fb = (F == 1) ? 0 : (F / 2 + r / P);
-  Lanes<T, NBITS, MAGIC> lanes;
+  Lanes<T, NBITS> lanes;
   lanes.init(8 - NBITS * (fa + 1), 8 - NBITS * (fb + 1));
 
   // this warp's k-chunk of every tile (the same for all tiles: all matrices share K)
@@ -509,13 +369,8 @@ __global__ void __launch_bounds__(256, SKCfg<T, NBITS, GS, MT, MAGIC>::MIN_CTAS)
           for (int mt = 0; mt < MT; ++mt) {
             const uint32_t b0 = (j == 0) ? ya[mt].x : (j == 1) ? ya[mt].z : (j == 2) ? yb[mt].x : yb[mt].z;
             const uint32_t b1 = (j == 0) ? ya[mt].y : (j == 1) ? ya[mt].w : (j == 2) ? yb[mt].y : yb[mt].w;
-            if (first) {
-              MM::mma0(Sg[mt], a0, a1, a2, a3, b0, b1);
-              MM::mma0(Xg[mt], MM::ONE2, MM::ONE2, MM::ONE2, MM::ONE2, b0, b1);
-            } else {
-              MM::mma(Sg[mt], a0, a1, a2, a3, b0, b1);
-              MM::mma(Xg[mt], MM::ONE2, MM::ONE2, MM::ONE2, MM::ONE2, b0, b1);
-            }
+            mma_m16n8k16<T>(Sg[mt], a0, a1, a2, a3, b0, b1, first);
+            mma_m16n8k16<T>(Xg[mt], MM::ONE2, MM::ONE2, MM::ONE2, MM::ONE2, b0, b1, first);
           }
           if (((us * 4 + j + 1) % MPG) == 0) {
             // a quantisation group is complete: tot += s*(Q - z*X), with lane value = OFF + q*V folded in
@@ -575,12 +430,12 @@ __global__ void __launch_bounds__(256, SKCfg<T, NBITS, GS, MT, MAGIC>::MIN_CTAS)
 // depends only on the activation is hoisted out of the per-tile loop: each warp stages ITS k-chunk of x once in shared
 // memory, already permuted to the lane pairing the bit-tricks produce ({k0,k2},{k1,k3}: no PRMT on the weights), and
 // sums it per quantisation group once (no all-ones MMA); the affine correction is applied to the single real column.
-// MR = 1 (experimental, HQQ_B200_D1_VARIANT=1042): scale/zero ride the cp.async ring at the same distance as the weights
-// (16-byte copies of the aligned block that holds this unit's 8 bytes) instead of register loads one unit ahead -- ncu showed
-// 18 % of all stall samples on the first use of those registers (DRAM latency under load exceeds one unit of work).
-template <typename T, int NBITS, int GS, int MAGIC, int ST, int MR = 0>
+// MR = 1: scale/zero ride the cp.async ring at the same distance as the weights (16-byte copies of the aligned block that holds
+// this unit's 8 bytes) instead of register loads one unit ahead -- ncu showed 18 % of all stall samples on the first use of
+// those registers (DRAM latency under load exceeds one unit of work).
+template <typename T, int NBITS, int GS, int ST, int MR = 0>
 struct D1Cfg {
-  static constexpr int F = 8 / NBITS, P = 16 / F, MPG = GS / 16, GPB = 256 / GS, MB = GPB * 2;
+  static constexpr int F = 8 / NBITS, P = 16 / F, MPG = GS / 16, GPB = 256 / GS;
   static constexpr int NWV = (F == 1) ? 8 : 4;
   static constexpr int W_BYTES = ST * NWV * 256 * 16;
   static constexpr int M_BYTES = (MR & 1) ? ST * 8 * 4 * 8 * 16 : 0;  // MR: [stage][warp][vector][row] 16-byte blocks; else registers
@@ -588,9 +443,9 @@ struct D1Cfg {
   static int smem(int K) { return W_BYTES + M_BYTES + P_BYTES + K * 2 + (K / GS) * 4; }
 };
 
-template <typename T, int NBITS, int GS, int MAGIC, int ST, int MC, int MR = 0>
+template <typename T, int NBITS, int GS, int ST, int MC, int MR = 0>
 __global__ void __launch_bounds__(256, MC) linear_decode1_kernel(const __grid_constant__ SKArgs a) {
-  using C = D1Cfg<T, NBITS, GS, MAGIC, ST, MR>;
+  using C = D1Cfg<T, NBITS, GS, ST, MR>;
   constexpr int F = C::F, P = C::P, MPG = C::MPG, GPB = C::GPB, NWV = C::NWV;
   using MM = MT16<T>;
   extern __shared__ __align__(16) uint8_t smem[];
@@ -604,7 +459,7 @@ __global__ void __launch_bounds__(256, MC) linear_decode1_kernel(const __grid_co
   const int r = lane >> 2, c = lane & 3;
   const int p = (F == 1) ? r : (r % P);
   const int fa = (F == 1) ? 0 : (r / P), fb = (F == 1) ? 0 : (F / 2 + r / P);
-  Lanes<T, NBITS, MAGIC> lanes;
+  Lanes<T, NBITS> lanes;
   lanes.init(8 - NBITS * (fa + 1), 8 - NBITS * (fb + 1));
 
   const int kb0 = a.KB * warp / 8, kb1 = a.KB * (warp + 1) / 8;
@@ -735,12 +590,8 @@ __global__ void __launch_bounds__(256, MC) linear_decode1_kernel(const __grid_co
       uint4 w0, w1;
       bool ok;
       do {
-#ifdef HQQ_EMU
-        memcpy(&w0, src, 16); memcpy(&w1, src + 4, 16);
-#else
-        asm volatile("ld.relaxed.sys.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(w0.x), "=r"(w0.y), "=r"(w0.z), "=r"(w0.w) : "l"(src) : "memory");
-        asm volatile("ld.relaxed.sys.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(w1.x), "=r"(w1.y), "=r"(w1.z), "=r"(w1.w) : "l"(src + 4) : "memory");
-#endif
+        w0 = ld_relaxed_sys_v4(src);
+        w1 = ld_relaxed_sys_v4(src + 4);
         ok = ((w0.x >> 16) == rtag) & ((w0.y >> 16) == rtag) & ((w0.z >> 16) == rtag) & ((w0.w >> 16) == rtag) &
              ((w1.x >> 16) == rtag) & ((w1.y >> 16) == rtag) & ((w1.z >> 16) == rtag) & ((w1.w >> 16) == rtag);
       } while (!ok);
@@ -764,7 +615,7 @@ __global__ void __launch_bounds__(256, MC) linear_decode1_kernel(const __grid_co
           for (int j = 0; j < 8; ++j) acc[j] += to_f32<T>(p8.v[j]);
         }
 #pragma unroll
-        for (int j = 0; j < 8; ++j) d.v[j] = from_f32_t<T>(acc[j]);
+        for (int j = 0; j < 8; ++j) d.v[j] = from_f32<T>(acc[j]);
         return true;
       }
       if (x2) { d = *reinterpret_cast<const Vec<T, 8>*>(x2 + k8); return true; }
@@ -797,11 +648,11 @@ __global__ void __launch_bounds__(256, MC) linear_decode1_kernel(const __grid_co
         const bool add_b = has_b && delta8(kb, db);
         if (add_a) {
 #pragma unroll
-          for (int j = 0; j < 8; ++j) va.v[j] = from_f32_t<T>(to_f32<T>(va.v[j]) + to_f32<T>(da.v[j]));
+          for (int j = 0; j < 8; ++j) va.v[j] = from_f32<T>(to_f32<T>(va.v[j]) + to_f32<T>(da.v[j]));
         }
         if (add_b) {
 #pragma unroll
-          for (int j = 0; j < 8; ++j) vb.v[j] = from_f32_t<T>(to_f32<T>(vb.v[j]) + to_f32<T>(db.v[j]));
+          for (int j = 0; j < 8; ++j) vb.v[j] = from_f32<T>(to_f32<T>(vb.v[j]) + to_f32<T>(db.v[j]));
         }
         *reinterpret_cast<Vec<T, 8>*>(xs + ka) = va;
         if (has_b) *reinterpret_cast<Vec<T, 8>*>(xs + kb) = vb;
@@ -830,7 +681,7 @@ __global__ void __launch_bounds__(256, MC) linear_decode1_kernel(const __grid_co
         Vec<T, 8> v = *reinterpret_cast<const Vec<T, 8>*>(xs + k8);
         const Vec<T, 8> g = (i == 0) ? g0 : (i == 1) ? g1 : *reinterpret_cast<const Vec<T, 8>*>(xw + k8);
 #pragma unroll
-        for (int j = 0; j < 8; ++j) v.v[j] = from_f32_t<T>(to_f32<T>(from_f32_t<T>(to_f32<T>(v.v[j]) * inv)) * to_f32<T>(g.v[j]));
+        for (int j = 0; j < 8; ++j) v.v[j] = from_f32<T>(to_f32<T>(from_f32<T>(to_f32<T>(v.v[j]) * inv)) * to_f32<T>(g.v[j]));
         put_permuted(k8, v);  // in place: every lane rewrites exactly the eight elements it read
       }
     } else {
@@ -845,7 +696,7 @@ __global__ void __launch_bounds__(256, MC) linear_decode1_kernel(const __grid_co
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
             const float f = to_f32<T>(v.v[j]);
-            v.v[j] = from_f32_t<T>(to_f32<T>(from_f32_t<T>(f / (1.0f + __expf(-f)))) * to_f32<T>(u.v[j]));
+            v.v[j] = from_f32<T>(to_f32<T>(from_f32<T>(f / (1.0f + __expf(-f)))) * to_f32<T>(u.v[j]));
           }
         }
         put_permuted(k8, v);
@@ -907,8 +758,7 @@ __global__ void __launch_bounds__(256, MC) linear_decode1_kernel(const __grid_co
           else lanes.extract_np(wa[j], a0, a1, a2, a3);
           const uint32_t b0 = (j == 0) ? xa.x : (j == 1) ? xa.z : (j == 2) ? xb.x : xb.z;
           const uint32_t b1 = (j == 0) ? xa.y : (j == 1) ? xa.w : (j == 2) ? xb.y : xb.w;
-          if (((us * 4 + j) % MPG) == 0) MM::mma0(Sg, a0, a1, a2, a3, b0, b1);
-          else MM::mma(Sg, a0, a1, a2, a3, b0, b1);
+          mma_m16n8k16<T>(Sg, a0, a1, a2, a3, b0, b1, ((us * 4 + j) % MPG) == 0);
           if (((us * 4 + j + 1) % MPG) == 0) {
             const int gi = (us * 4 + j) / MPG;
             const float X = xsum[kb * GPB + gi];
@@ -939,7 +789,7 @@ __global__ void __launch_bounds__(256, MC) linear_decode1_kernel(const __grid_co
           const int n = ff * tg.step + prow;
           const float f = to_f32<T>(MM::cvt(ag, tg.bias, n));
           const float u = to_f32<T>(MM::cvt(au, tu.bias, n));
-          tg.y[n] = from_f32_t<T>(to_f32<T>(from_f32_t<T>(f / (1.0f + __expf(-f)))) * u);
+          tg.y[n] = from_f32<T>(to_f32<T>(from_f32<T>(f / (1.0f + __expf(-f)))) * u);
         }
         continue;
       }
@@ -952,16 +802,16 @@ __global__ void __launch_bounds__(256, MC) linear_decode1_kernel(const __grid_co
         const int n = ff * t.step + prow;
         MM::st(t.y, n, acc, t.bias, n);
         if (a.peer_data[0] || t.ytag) {
-          const T pv = from_f32_t<T>(acc);
+          const T pv = from_f32<T>(acc);
           const uint32_t word = (send_tag << 16) | (uint32_t)(*reinterpret_cast<const unsigned short*>(&pv));
           if (a.peer_data[0]) {
             // scatter the (bias-free) partial over NVLink as one tagged word per value: slot [parity][rank][n] on every rank
             const size_t off = ((size_t)send_par * a.tp + a.rank) * t.N + n;
 #pragma unroll
             for (int dst = 0; dst < 8; ++dst)
-              if (dst < a.tp) HQQ_ST_RELAXED_SYS(a.peer_data[dst] + off, word);
+              if (dst < a.tp) st_relaxed_sys_u32(a.peer_data[dst] + off, word);
           }
-          if (t.ytag) HQQ_ST_RELAXED_SYS(t.ytag + (size_t)send_par * t.N + n, word);
+          if (t.ytag) st_relaxed_sys_u32(t.ytag + (size_t)send_par * t.N + n, word);
         }
       }
     }
@@ -970,123 +820,39 @@ __global__ void __launch_bounds__(256, MC) linear_decode1_kernel(const __grid_co
 }
 
 // ---------------------------------------------------------------------------------------------------------
-static int magic_mode() {
-  HQQ_ENV_KNOB(mode, ([] { const char* e = getenv("HQQ_B200_GEMV_MAGIC"); return (e && !strcmp(e, "subnormal")) ? MAGIC_SUBNORMAL : MAGIC_OFFSET; })());
-  return mode;
-}
-
-// Function attributes (opt-in dynamic shared memory) and SM counts belong to ONE device: every cache below is indexed by the
-// calling thread's current device, so layers living on several GPUs of one process each get their own setup.
-constexpr int kMaxDevices = 64;
-static int cur_device() {
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= kMaxDevices) dev = 0;
-  return dev;
-}
-
-static int sm_count() {
-  static int n[kMaxDevices] = {};
-  const int dev = cur_device();
-  if (!n[dev]) {
-    if (cudaDeviceGetAttribute(&n[dev], cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n[dev] <= 0) n[dev] = kNumSMs;
-  }
-  return n[dev];
-}
-
-template <typename T, int NBITS, int GS, int MT, int MAGIC>
-static int grid_for_kernel(int* grid_out) {
-  using C = SKCfg<T, NBITS, GS, MT, MAGIC>;
+// Persistent CTAs: every CTA slot of every SM (measured on the B200: the kernel is bound per SM, so filling every slot beats
+// fewer, equally loaded CTAs), or one CTA per tile when there are fewer tiles.
+template <typename T, int NBITS, int GS, int MT>
+static int launch_sk(SKArgs& a, cudaStream_t st) {
+  using C = SKCfg<T, NBITS, GS, MT>;
+  constexpr auto k = linear_small_kernel<T, NBITS, GS, MT>;
   static int grids[kMaxDevices] = {};
   int& grid = grids[cur_device()];
   if (!grid) {
-    auto k = linear_small_kernel<T, NBITS, GS, MT, MAGIC>;
-    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM);
-    HQQ_REQUIRE(e == cudaSuccess, HQQ_E_CUDA, "hqq_b200_linear_fwd: cannot reserve %d bytes of shared memory: %s", C::SMEM, cudaGetErrorString(e));
+    const int rc = reserve_smem<k>(C::SMEM);
+    if (rc) return rc;
     int occ = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k, 256, C::SMEM);
+    const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k, 256, C::SMEM);
     HQQ_REQUIRE(e == cudaSuccess && occ > 0, HQQ_E_CUDA, "hqq_b200_linear_fwd: occupancy query failed: %s", cudaGetErrorString(e));
     if (occ > 2) occ = 2;
     grid = sm_count() * occ;
   }
-  *grid_out = grid;
-  return HQQ_OK;
+  return launch_pdl("hqq_b200_linear_fwd/small", k, dim3((unsigned)(a.total_tiles < grid ? a.total_tiles : grid)), dim3(256), C::SMEM, st,
+                    pdl_enabled(), a);
 }
 
-// Persistent CTAs take tiles round-robin, so a grid that does not divide the tile count leaves most CTAs idle during the
-// last round (896 tiles on 296 CTAs = 3.03 -> 4 rounds, 76 %).  The kernel is bound by aggregate HBM bandwidth, not by
-// per-SM work, so it is better to launch fewer, equally loaded CTAs: pick g in [max_grid/2, max_grid] maximising
-// tiles / (ceil(tiles/g) * g); ties go to the larger grid.
-static int balanced_grid(int tiles, int max_grid) {
-  if (tiles <= max_grid) return tiles;
-  HQQ_ENV_KNOB(mode, ([] { const char* e = getenv("HQQ_B200_BALANCED_GRID"); return (e && e[0] == '1') ? 1 : 0; })());
-  if (!mode) return max_grid;  // measured on B200: the kernel is bound per SM, so filling every CTA slot wins
-  int best = max_grid;
-  double best_eff = 0.0;
-  for (int g = max_grid; g >= max_grid / 2; --g) {
-    const int rounds = (tiles + g - 1) / g;
-    const double eff = (double)tiles / ((double)rounds * g);
-    if (eff > best_eff + 1e-9) { best_eff = eff; best = g; }
-  }
-  return best;
-}
-
-static bool pdl_enabled() {
-  HQQ_ENV_KNOB(on, ([] { const char* e = getenv("HQQ_B200_PDL"); return (e && e[0] == '0') ? 0 : 1; })());
-  return on == 1;
-}
-
-template <typename T, int NBITS, int GS, int MT, int MAGIC>
-static int launch_sk(SKArgs& a, cudaStream_t st) {
-  using C = SKCfg<T, NBITS, GS, MT, MAGIC>;
-  int grid = 0;
-  int rc = grid_for_kernel<T, NBITS, GS, MT, MAGIC>(&grid);
-  if (rc) return rc;
-  grid = balanced_grid(a.total_tiles, grid);
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(256);
-  cfg.dynamicSmemBytes = C::SMEM;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, linear_small_kernel<T, NBITS, GS, MT, MAGIC>, a);
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  HQQ_REQUIRE(e == cudaSuccess, HQQ_E_CUDA, "hqq_b200_linear_fwd/small: CUDA launch failed: %s", cudaGetErrorString(e));
-  return HQQ_OK;
-}
-
-template <typename T, int NBITS, int GS, int MAGIC, int ST, int MC, int MR = 0>
+template <typename T, int NBITS, int GS, int ST, int MC, int MR = 0>
 static int launch_d1(SKArgs& a, cudaStream_t st) {
-  using C = D1Cfg<T, NBITS, GS, MAGIC, ST, MR>;
-  static int max_smems[kMaxDevices] = {};
-  int& max_smem = max_smems[cur_device()];
+  using C = D1Cfg<T, NBITS, GS, ST, MR>;
+  constexpr auto k = linear_decode1_kernel<T, NBITS, GS, ST, MC, MR>;
   const int smem = C::smem(a.K);
-  auto k = linear_decode1_kernel<T, NBITS, GS, MAGIC, ST, MC, MR>;
-  if (smem > max_smem) {
-    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    HQQ_REQUIRE(e == cudaSuccess, HQQ_E_CUDA, "hqq_b200_linear_fwd: cannot reserve %d bytes of shared memory: %s", smem, cudaGetErrorString(e));
-    max_smem = smem;
-  }
+  const int rc = reserve_smem<k>(smem);
+  if (rc) return rc;
   int per_sm = MC;
   while (per_sm > 1 && (smem + 1024) * per_sm > 227 * 1024) --per_sm;
-  int grid = balanced_grid(a.total_tiles, sm_count() * per_sm);
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(256);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, k, a);
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  HQQ_REQUIRE(e == cudaSuccess, HQQ_E_CUDA, "hqq_b200_linear_fwd/decode1: CUDA launch failed: %s", cudaGetErrorString(e));
-  return HQQ_OK;
+  const int grid = sm_count() * per_sm;
+  return launch_pdl("hqq_b200_linear_fwd/decode1", k, dim3((unsigned)(a.total_tiles < grid ? a.total_tiles : grid)), dim3(256), smem, st,
+                    pdl_enabled(), a);
 }
 
 static bool d1_enabled() {
@@ -1094,53 +860,46 @@ static bool d1_enabled() {
   return on == 1;
 }
 
-template <typename T, int NBITS, int GS, int MAGIC>
+template <typename T, int NBITS, int GS>
 static int sk_mt(SKArgs& a, cudaStream_t st) {
   if (a.M == 1 && a.K <= 16384 && d1_enabled()) {
-    if (NBITS == 8) return launch_d1<T, NBITS, GS, MAGIC, 2, 2>(a, st);
+    if (NBITS == 8) return launch_d1<T, NBITS, GS, 2, 2>(a, st);
     // scale/zero ride the cp.async ring at the weights' distance (MR = 1) whenever the ring's aligned 16-byte copies are legal;
-    // measured on the B200 (round 2, profiles/r2_d1_variants.txt): 1.70 ms per token against 1.91 ms with register loads one
+    // measured on the B200 (round 2, profiles/r2_variant_sweep.log): 1.70 ms per token against 1.91 ms with register loads one
     // unit ahead, bit-identical outputs.  evict-first hints, a third CTA per SM, L2 prefetch under the dependency wait and
     // cross-launch weight prefetch were measured in the same run, were not faster, and are gone.
     if constexpr (GS == 64 && NBITS != 8) {
       if (a.K % 512 == 0) {
         bool ok = true;  // the ring copies aligned 16-byte blocks: every group row must start on one
         for (int i = 0; i < a.nprob; ++i) ok = ok && aligned(a.p[i].scale, 16) && aligned(a.p[i].zero, 16);
-        if (ok) return launch_d1<T, NBITS, GS, MAGIC, 4, 2, 1>(a, st);
+        if (ok) return launch_d1<T, NBITS, GS, 4, 2, 1>(a, st);
       }
     }
-    return launch_d1<T, NBITS, GS, MAGIC, 4, 2>(a, st);
+    return launch_d1<T, NBITS, GS, 4, 2>(a, st);
   }
-  if (a.M <= 8) return launch_sk<T, NBITS, GS, 1, MAGIC>(a, st);
-  if (a.M <= 16) return launch_sk<T, NBITS, GS, 2, MAGIC>(a, st);
-  return launch_sk<T, NBITS, GS, 4, MAGIC>(a, st);
+  if (a.M <= 8) return launch_sk<T, NBITS, GS, 1>(a, st);
+  if (a.M <= 16) return launch_sk<T, NBITS, GS, 2>(a, st);
+  return launch_sk<T, NBITS, GS, 4>(a, st);
 }
 
-template <typename T, int NBITS, int MAGIC>
+template <typename T, int NBITS>
 static int sk_gs(SKArgs& a, int gs, cudaStream_t st) {
   switch (gs) {
-    case 64: return sk_mt<T, NBITS, 64, MAGIC>(a, st);
-    case 128: return sk_mt<T, NBITS, 128, MAGIC>(a, st);
+    case 64: return sk_mt<T, NBITS, 64>(a, st);
+    case 128: return sk_mt<T, NBITS, 128>(a, st);
   }
   return HQQ_E_UNSUPPORTED;
 }
 
 template <typename T>
 static int sk_bits(SKArgs& a, int gs, int nbits, cudaStream_t st) {
-  const bool sub = std::is_same<T, __half>::value && magic_mode() == MAGIC_SUBNORMAL;
   switch (nbits) {
     case 8:
-      if constexpr (std::is_same<T, __half>::value) return sub ? sk_gs<T, 8, MAGIC_SUBNORMAL>(a, gs, st) : sk_gs<T, 8, MAGIC_OFFSET>(a, gs, st);
-      else return HQQ_E_UNSUPPORTED;
-    case 4:
-      if constexpr (std::is_same<T, __half>::value) return sub ? sk_gs<T, 4, MAGIC_SUBNORMAL>(a, gs, st) : sk_gs<T, 4, MAGIC_OFFSET>(a, gs, st);
-      else return sk_gs<T, 4, MAGIC_OFFSET>(a, gs, st);
-    case 2:
-      if constexpr (std::is_same<T, __half>::value) return sub ? sk_gs<T, 2, MAGIC_SUBNORMAL>(a, gs, st) : sk_gs<T, 2, MAGIC_OFFSET>(a, gs, st);
-      else return sk_gs<T, 2, MAGIC_OFFSET>(a, gs, st);
-    case 1:
-      if constexpr (std::is_same<T, __half>::value) return sub ? sk_gs<T, 1, MAGIC_SUBNORMAL>(a, gs, st) : sk_gs<T, 1, MAGIC_OFFSET>(a, gs, st);
-      else return sk_gs<T, 1, MAGIC_OFFSET>(a, gs, st);
+      if constexpr (std::is_same<T, __half>::value) return sk_gs<T, 8>(a, gs, st);
+      else return HQQ_E_UNSUPPORTED;  // 8-bit levels need the fp16 lanes
+    case 4: return sk_gs<T, 4>(a, gs, st);
+    case 2: return sk_gs<T, 2>(a, gs, st);
+    case 1: return sk_gs<T, 1>(a, gs, st);
   }
   return HQQ_E_UNSUPPORTED;
 }

@@ -51,9 +51,10 @@ def rewrite(src: str) -> str:
 
 def digest() -> str:
     h = hashlib.sha256()
-    files = [os.path.join(CSRC, f) for f in SOURCES + ["common.cuh", "linear_internal.cuh"]] + [os.path.join(ROOT, "include", "hqq_b200.h"), __file__,
-                                                                        os.path.join(HERE, "include", "cuda_runtime.h"),
-                                                                        os.path.join(HERE, "emu_runtime.cpp")]
+    headers = sorted(f for f in os.listdir(CSRC) if f.endswith(".cuh"))  # every header: a new one must not leave a stale library
+    files = [os.path.join(CSRC, f) for f in SOURCES + headers] + [os.path.join(ROOT, "include", "hqq_b200.h"), __file__,
+                                                                  os.path.join(HERE, "include", "cuda_runtime.h"),
+                                                                  os.path.join(HERE, "emu_runtime.cpp")]
     for f in files:
         with open(f, "rb") as fh:
             h.update(fh.read())

@@ -1,7 +1,6 @@
 """TEST INFRASTRUCTURE ONLY: `hqq_b200_reload_env()` on the emulated library -- the HQQ_B200_* knobs are cached per process and
 parsed again only after a reload.  Observable without a GPU: HQQ_B200_DECODE1=0 removes the one-token kernel, and with it the fused
-activation prologues (`hqq_b200_decode_linear_fwd` with x_op != 0 answers HQQ_E_UNSUPPORTED); HQQ_B200_D1_VARIANT selects kernels
-that must stay bit-identical.  Prints one JSON line."""
+activation prologues (`hqq_b200_decode_linear_fwd` with x_op != 0 answers HQQ_E_UNSUPPORTED).  Prints one JSON line."""
 import ctypes
 import json
 import os
