@@ -204,10 +204,18 @@ def _on(dev: torch.device):
     return torch.cuda.device(dev)
 
 
+def _aligned16(t: torch.Tensor) -> torch.Tensor:
+    """`t`, or a fresh contiguous copy of it when its data pointer is not 16-byte aligned.  The forward kernels load
+    activations (and the dense GEMM its weight) in 16-byte vectors or through TMA and reject other pointers; a contiguous
+    view at an element offset (x[1:] of a flat buffer) is still a valid activation, so it is copied instead."""
+    return t if t.data_ptr() % 16 == 0 else t.clone(memory_format=torch.contiguous_format)
+
+
 def linear_fwd(x2d: torch.Tensor, W_q: torch.Tensor, scale: torch.Tensor, zero: torch.Tensor, bias, N: int, K: int,
                group_size: int, nbits: int, axis: int, out: torch.Tensor | None = None) -> torch.Tensor | None:
     """y = x2d @ dequantize(W_q).T (+ bias) through the fused kernels; returns None when no fused kernel covers
     the configuration (caller then uses dequantize + matmul)."""
+    x2d = _aligned16(x2d)
     dtype = x2d.dtype
     M = x2d.shape[0]
     lib = load()
@@ -236,7 +244,7 @@ def dense_gemm(x2d: torch.Tensor, W: torch.Tensor, bias=None, out: torch.Tensor 
     N = W.shape[0]
     if code not in (DTYPE_CODE[torch.float16], DTYPE_CODE[torch.bfloat16]) or W.dtype != x2d.dtype or W.shape[1] != K or K % 8:
         return None
-    x2d, W = x2d.contiguous(), W.contiguous()
+    x2d, W = _aligned16(x2d.contiguous()), _aligned16(W.contiguous())
     y = out if out is not None else torch.empty((M, N), dtype=x2d.dtype, device=x2d.device)
     with _on(x2d.device):
         rc = load().hqq_b200_dense_gemm(ptr(x2d), ptr(W), ptr(bias), ptr(y), M, N, K, code, stream_ptr(x2d.device))
@@ -276,6 +284,7 @@ def linear_fwd_multi(x2d: torch.Tensor, layers, outs=None):
             return None
         Ns.append(N)
     dev = x2d.device
+    x2d = _aligned16(x2d)
     if outs is None:
         outs = [torch.empty((M, N), dtype=dtype, device=dev) for N in Ns]
     VP = ctypes.c_void_p * n

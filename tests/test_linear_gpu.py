@@ -5,6 +5,11 @@ Stated tolerance (BASELINE north_star "within a stated fp tolerance"): relative 
 ||y - y_ref|| / ||y_ref|| <= 2e-3 for float16 and <= 1e-2 for bfloat16.  The fused kernels keep the integer levels
 exact and apply scale/zero in float32, so they differ from the reference only by the reference's own fp16/bf16
 rounding of W_r and by accumulation order.
+
+A norm over a whole output cannot see a fault in a few elements.  tests/test_linear_bounds_gpu.py holds every route, in both
+dtypes, to a per-element bound around a float64 reference, |y - y*| <= ulp_T + c * 2^-24 * (accumulation mass), and checks the
+exact identities bit for bit: route 2 == dense GEMM over layer.dequantize() without split-K, y(x, b) == y(x, None) + b, and
+split-K results independent of the second-pass variant and of the workspace contents.
 """
 import numpy as np
 import pytest
